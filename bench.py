@@ -7,7 +7,8 @@
 Metric (BASELINE.json): frames/sec and real-time factor.  Workloads (BASELINE.json configs, 1-based like BASELINE.md):
   --config 2 (default)  FullSubNet+ default config/inference.toml, 64 x 3 s clips per GPU per step (weak scaling; N = 8 is configs[2])
   --config 4            streaming: fullsubnet.Model + cumulative_laplace_norm, look_ahead 2, one 30 s clip frame by frame through the
-                        step API; per-frame latency p50 / p99 (+ the offline forwards of both models on the same clip)
+                        step API, one frame per step (--steps 1876 = the whole clip); per-frame latency p50 / p99 (+ the offline
+                        forwards of both models on the same clip)
   --config 5            large model: num_freqs 513 (n_fft 1024, hop 512), hidden 512, 3-layer LSTMs, 32 x 3 s clips
 
 Configs 2 / 5, what one "step" is (identical at every N, so the driver's scaling efficiency compares like with like):
@@ -20,7 +21,9 @@ Configs 2 / 5, what one "step" is (identical at every N, so the driver's scaling
   extras    forward_only (plain fsn_model_forward loop, the round-1 `value`), e2e_cabi (fsn_model_forward_host_async loop: mask to
             host, the round-1 `e2e`), cudnn_baseline (the reference model on the same B200 through stock PyTorch / cuDNN),
             cpu_baseline (+ .concurrent: as many B=1 workers as the host has cores for).
-Prints ONE JSON line on rank 0.
+Prints ONE JSON line on rank 0.  ``--dump-outputs DIR`` then writes what the timed path (`value`) returned in its last step as
+DIR/<name>.npy in float32 (configs 2 / 5: ``enhanced`` [N, samples], the waveforms of every rank; config 4: ``mask`` [B, 2, F], the
+mask the last step returned), at most 64 MB in all; the inputs and the weights are seeded, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -32,9 +35,11 @@ import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
+sys.dont_write_bytecode = True                  # the benchmark leaves the tree as it found it (it may be read-only)
 sys.path[:0] = [ROOT, os.path.join(ROOT, "fullsubnet-plus_b200")]
 
 SR = 16000
+DUMP_BYTES = 64 * 10 ** 6                       # --dump-outputs: budget of all files together
 
 
 # ------------------------------------------------------------------------------------------------------------------
@@ -296,7 +301,7 @@ def reference_arm(args, w, state):
 # ------------------------------------------------------------------------------------------------------------------
 # product arm, configs 2 / 5
 # ------------------------------------------------------------------------------------------------------------------
-def product_batched(args, w, model, state, rank, local_rank, world, make_model):
+def product_batched(args, w, model, state, rank, local_rank, world, make_model, outputs):
     import torch
     import torch.distributed as dist
     from fsnplus_b200.synth import synth_clips
@@ -360,6 +365,7 @@ def product_batched(args, w, model, state, rank, local_rank, world, make_model):
         time.sleep(0.3)
     ms_step, t0, t1 = timed(lambda i: pipe.push(Xs[i % NSETS]), K, max(W, pipe.NSLOT + 1), drain=pipe.flush)   # warm-up fills every ring slot (allocations)
     host_ms = timed.host_ms
+    outputs["enhanced"] = pipe.last.cpu().numpy()                 # the last timed step's waveforms (all ranks' when gathered)
     clocks = sampler.stop(t0, t1) if sampler else None
     lstm_ms = [x for x in model.lstm_ms_history(min(K, 32)) if x > 0]
     fps = world * B * T / (ms_step * 1e-3)
@@ -452,7 +458,7 @@ def product_batched(args, w, model, state, rank, local_rank, world, make_model):
 # ------------------------------------------------------------------------------------------------------------------
 # product arm, config 4 (streaming)
 # ------------------------------------------------------------------------------------------------------------------
-def product_streaming(args, w, model, state, rank, local_rank, world):
+def product_streaming(args, w, model, state, rank, local_rank, world, outputs):
     import numpy as np
     import torch
     from fsnplus_b200.synth import synth_clips
@@ -467,7 +473,9 @@ def product_streaming(args, w, model, state, rank, local_rank, world):
     T = mag.shape[-1]
     frames = [mag[:, :, t].contiguous() for t in range(T)]
     hframes = [f.cpu().pin_memory() for f in frames]
-    K = T if args.steps <= 5 else min(T, args.steps)              # default: the whole 30 s clip
+    K = args.steps
+    if K > T:
+        raise SystemExit(f"--steps {K}: the {w['clip_s']:.0f} s clip has {T} frames (one frame per step)")
 
     def run(host):
         st = StreamingFullSubNet(model, batch_size=B, device=dev)
@@ -495,6 +503,7 @@ def product_streaming(args, w, model, state, rank, local_rank, world):
             lat.append((time.perf_counter() - t0) * 1e3)
         if not host:
             dev_ms = [a.elapsed_time(b) for a, b in evs]
+            outputs["mask"] = y.cpu().numpy() if y is not None else None
         st.close()
         return np.array(lat), np.array(dev_ms)
 
@@ -633,6 +642,22 @@ def cpu_baseline(args, w, state):
     return out
 
 
+def dump_outputs(dirname, arrays):
+    """Write each array as dirname/<name>.npy in float32.  Beyond DUMP_BYTES in all, every array keeps a fixed, seeded sample of
+    its rows (first axis, in order) in proportion to its size; the same shapes always give the same sample."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v, dtype=np.float32) for k, v in arrays.items() if v is not None}
+    if not arrays:
+        raise SystemExit("--dump-outputs: the timed path returned nothing in its last step")
+    total = sum(a.nbytes for a in arrays.values())
+    os.makedirs(dirname, exist_ok=True)
+    for name, a in arrays.items():
+        if total > DUMP_BYTES:
+            keep = max(1, DUMP_BYTES * a.shape[0] // total)
+            a = a[np.sort(np.random.default_rng(0).choice(a.shape[0], keep, replace=False))]
+        np.save(os.path.join(dirname, name + ".npy"), a)
+
+
 # ------------------------------------------------------------------------------------------------------------------
 def main():
     ap = argparse.ArgumentParser()
@@ -649,7 +674,12 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-cudnn-baseline", action="store_true")
     ap.add_argument("--no-overlap-experiment", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs as DIR/<name>.npy (float32, <= 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the B200 path (--impl b200)")
 
     import torch
     rank = int(os.environ.get("RANK", "0"))
@@ -677,10 +707,13 @@ def main():
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     model = model.to(dev)
+    outputs = {}
     if w["id"] == 4:
-        line = product_streaming(args, w, model, state, rank, local_rank, world)
+        line = product_streaming(args, w, model, state, rank, local_rank, world, outputs)
     else:
-        line = product_batched(args, w, model, state, rank, local_rank, world, make_model)
+        line = product_batched(args, w, model, state, rank, local_rank, world, make_model, outputs)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     if rank == 0:
         if world == 1 and not args.no_cudnn_baseline:
             try:

@@ -177,6 +177,7 @@ class EnhancePipeline:
         ring = lambda: [None] * self.NSLOT
         self.inbuf, self.outbuf, self.post_done, self.host_out, self.gathered = ring(), ring(), ring(), ring(), ring()
         self.results = []
+        self.last = None                          # result of the most recently finished batch (kept or not)
 
     def _slot(self, slot, B, F, T):
         if self.inbuf[slot] is None or tuple(self.inbuf[slot][0].shape) != (B, 1, F, T):
@@ -211,6 +212,7 @@ class EnhancePipeline:
             if self.post_done[slot] is None:
                 self.post_done[slot] = torch.cuda.Event()
             self.post_done[slot].record(self.post)
+        self.last = res
         if self.keep:
             self.results.append(res)
 

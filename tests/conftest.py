@@ -1,3 +1,4 @@
+import glob
 import os
 import sys
 
@@ -31,5 +32,9 @@ def golden():
     import numpy as np
 
     def load(name):
-        return dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+        """Arrays of <name>.npz, merged with those of its parts <name>.<part>.npz (a fixture split to keep files small)."""
+        d = dict(np.load(os.path.join(GOLDEN, name + ".npz")))
+        for part in sorted(glob.glob(os.path.join(GOLDEN, glob.escape(name) + ".*.npz"))):
+            d.update(np.load(part))
+        return d
     return load

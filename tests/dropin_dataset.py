@@ -1,4 +1,4 @@
-"""Inference dataset for tests/test_reference_dropin.py: the interface of the reference's
+"""Inference dataset through which tests/golden/make_golden.py feeds clips to the reference's inferencer: the interface of its
 fullsubnet/dataset/dataset_inference.py:10-45 (``__getitem__`` -> (float32 waveform, basename)) without librosa: the clips come
 from one .npy file."""
 import numpy as np

@@ -1,9 +1,9 @@
 """Generate the committed golden vectors from the UNMODIFIED reference.
 
-Run in the authoring container only (needs /root/reference, which does not
-exist on the GPU box):
+Run where a checkout of the reference is available (found by
+oracle/ref_loader.py); the tests only read the fixtures:
 
-    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py
+    PYTHONDONTWRITEBYTECODE=1 python tests/golden/make_golden.py [causal|inferencer]
 
 The reference is imported read-only (librosa stubbed, SURVEY.md 8c), loaded with
 the deterministic numpy parameters of ``oracle.fsn_oracle.make_params_*`` through
@@ -14,15 +14,15 @@ float32 ``.npz`` fixtures next to this script.
 """
 import os
 import sys
-import types
 
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-sys.modules.setdefault("librosa", types.ModuleType("librosa"))
-sys.path[:0] = ["/root/reference", "/root/reference/speech_enhance"]
+from oracle import ref_loader  # noqa: E402
+
+ref_loader.setup()                                  # the reference on sys.path, librosa / soundfile stubbed (never called)
 
 import torch  # noqa: E402
 
@@ -152,8 +152,10 @@ def main():
                             length=clips.shape[1]).numpy()
             dref = ref_decompress(torch.from_numpy(out).permute(0, 2, 3, 1)).numpy()
             print("   decompress oracle-vs-ref:", O.rel_l2(O.decompress_cIRM(out).transpose(0, 2, 3, 1), dref))
-            save(tag, mag=mag, real=real, imag=imag, out=out, fb_in=fb_in, fb_out=fb_out, enhanced=enh,
-                 seed=0, lstm_scale=scale)
+            # three files, each under 1 MB; tests/conftest.py merges "<name>.<part>.npz" into "<name>"
+            save(tag, mag=mag, real=real, imag=imag, seed=0, lstm_scale=scale)
+            save(tag + ".outputs", out=out, enhanced=enh)
+            save(tag + ".stages", fb_in=fb_in, fb_out=fb_out)
         else:
             save(tag, out=out, seed=0, lstm_scale=scale)
 
@@ -239,6 +241,43 @@ def main():
     save("lstm3_small", x=x, out=y, seed=12)
 
 
+def main_inferencer():
+    """The reference's own inferencer (tools/inference.py:11-18: initialize_module(inferencer path) -> Inferencer(config, ckpt,
+    out)()) with the reference model on the CPU, driven by its shipped config/inference.toml and a reference-format checkpoint
+    of the seed-0 parameters: the int16 waveforms it writes for synthetic clips 0 and 1, the model calls it makes, and the
+    state-dict keys and shapes of the reference class built from that TOML.  tests/test_reference_dropin.py checks the
+    drop-in class against these."""
+    import tempfile
+    import toml
+    from oracle import ref_loader
+    root = ref_loader.reference_root()
+    _, sf = ref_loader._stubs()
+    sys.path.insert(0, os.path.dirname(HERE))                              # tests/dropin_dataset.py
+    from audio_zen.utils import initialize_module
+    cfg = toml.load(os.path.join(root, "config", "inference.toml"))
+    params = O.make_params_plus(O.default_plus_config(), seed=0)
+    calls = []
+    with tempfile.TemporaryDirectory() as tmp:
+        np.save(os.path.join(tmp, "clips.npy"), O.synth_clips(2).astype(np.float32))
+        cfg["dataset"] = {"path": "dropin_dataset.Dataset", "args": {"npy_path": os.path.join(tmp, "clips.npy"), "sr": 16000}}
+        torch.save({"model": {k: torch.from_numpy(v) for k, v in params.items()}, "epoch": 7}, os.path.join(tmp, "ckpt.tar"))
+        inferencer = initialize_module(cfg["inferencer"]["path"], initialize=False)(cfg, os.path.join(tmp, "ckpt.tar"), os.path.join(tmp, "out"))
+        inferencer.model.register_forward_hook(lambda m, i, o: calls.append([list(x.shape) for x in i] + [list(o.shape)]))
+        sf.written.clear()
+        inferencer()
+        written = {os.path.relpath(k, os.path.join(tmp, "out")): v for k, v in sf.written.items()}
+    names = sorted(written)
+    assert names == ["enhanced_0007/clip0.wav", "enhanced_0007/clip1.wav"], names
+    assert all(written[n][1] == 16000 and written[n][0].dtype == np.int16 for n in names)
+    sd = FullSubNet_Plus(**cfg["model"]["args"]).state_dict()
+    shapes = np.full((len(sd), 4), -1, np.int64)
+    for j, v in enumerate(sd.values()):
+        shapes[j, :v.dim()] = v.shape
+    print(f"reference inferencer: {len(calls)} model calls {calls[0]}, wrote {names}")
+    save("reference_inferencer", pcm=np.stack([written[n][0] for n in names]), files=np.array(names),
+         model_calls=np.array(calls, np.int64), state_dict_keys=np.array(list(sd)), state_dict_shapes=shapes, seed=0)
+
+
 def main_causal():
     """Round 2: the causal FullSubNet+ variant (SURVEY.md 8f rank 2): TCNBlock(causal=True) in all three full-band models."""
     ccfg = dict(small_plus_cfg(), causal_tcn=True)
@@ -256,6 +295,9 @@ def main_causal():
 if __name__ == "__main__":
     if "causal" in sys.argv[1:]:
         main_causal()
+    elif "inferencer" in sys.argv[1:]:
+        main_inferencer()
     else:
         main()
         main_causal()
+        main_inferencer()

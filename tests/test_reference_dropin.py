@@ -1,90 +1,105 @@
-"""The drop-in claim of INTEGRATION.md, executed: the reference's OWN loader and inferencer code (unmodified, imported from
-/root/reference here or from the verbatim copy oracle/_ref/ on the GPU box) driving ``fsnplus_b200.model.FullSubNet_Plus`` after
-changing ONE string of config/inference.toml (``[model] path``).
+"""The drop-in claim of INTEGRATION.md: the reference's loader and inferencer steps, driven by its shipped config/inference.toml
+after changing ONE string (``[model] path``), work unchanged with ``fsnplus_b200.model.FullSubNet_Plus``.
 
-  reference code on this path: audio_zen/utils.py:63-99 (initialize_module), audio_zen/inferencer/base_inferencer.py:22-60,97-110
-  (_load_model: initialize_module + torch.load + load_state_dict + .to(device) + .eval()), :133-160 (__call__: int16 scaling,
-  sf.write) and fullsubnet_plus/inferencer/inferencer.py:140-165 (mag_complex_full_band_crm_mask).
+  reference code on this path: audio_zen/utils.py:63-99 (initialize_module: dotted path -> class(**args)),
+  audio_zen/inferencer/base_inferencer.py:97-110 (_load_model: initialize_module + torch.load + load_state_dict + .to(device) +
+  .eval()), :133-160 (__call__: one clip per call, int16 scaling) and fullsubnet_plus/inferencer/inferencer.py:140-165
+  (mag_complex_full_band_crm_mask).
 
-CPU test: everything up to the forward (construction from the shipped TOML's [model.args], strict checkpoint load, eval) and the
-documented error on CPU tensors.  GPU test: the whole reference inferencer loop with the model on the B200, its written int16
-waveform compared with the golden waveform of the all-reference pipeline.
+What the reference did on this path is stored in tests/golden/reference_inferencer.npz (tests/golden/make_golden.py
+``inferencer``): the state-dict keys and shapes of the reference class built from that TOML, the model calls its inferencer
+makes, and the int16 waveforms it writes for synthetic clips 0 and 1 with the reference model and the same checkpoint.
+
+CPU test: everything up to the forward (construction from the TOML's [model.args], strict checkpoint load, eval, the reference
+class's keys and shapes) and the documented error on CPU tensors.  GPU test: the inferencer's per-clip loop with the model on
+the B200, its int16 waveforms compared with those the all-reference inferencer wrote.
 """
+import importlib
 import os
-import sys
 
 import numpy as np
 import pytest
 import torch
 
 from oracle import fsn_oracle as O
-from oracle import ref_loader
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-needs_ref = pytest.mark.skipif(not ref_loader.available(), reason="reference not available (neither /root/reference nor oracle/_ref)")
+REF_TOML = os.path.join(HERE, "golden", "inference_reference.toml")
 
 
-def _config(tmp_path, clips):
-    import toml
-    root = ref_loader.setup()
-    cfg = toml.load(os.path.join(root, "config", "inference.toml"))
+def _config(tmp_path):
+    from fsnplus_b200.tools import inference as T
+    cfg = T.load_toml(REF_TOML)
     assert cfg["model"]["path"] == "fullsubnet_plus.model.fullsubnet_plus.FullSubNet_Plus"
     cfg["model"]["path"] = "fsnplus_b200.model.FullSubNet_Plus"          # <- the one-string swap of INTEGRATION.md
-    if HERE not in sys.path:
-        sys.path.insert(0, HERE)
-    np.save(tmp_path / "clips.npy", clips)
-    cfg["dataset"] = {"path": "dropin_dataset.Dataset", "args": {"npy_path": str(tmp_path / "clips.npy"), "sr": 16000}}
     ckpt = tmp_path / "ckpt.tar"
     params = O.make_params_plus(O.default_plus_config(), seed=0)
     torch.save({"model": {k: torch.from_numpy(v) for k, v in params.items()}, "epoch": 7}, ckpt)
     return cfg, ckpt
 
 
-@needs_ref
-def test_reference_loader_builds_and_loads_the_dropin_class(tmp_path, built_lib):
-    cfg, ckpt = _config(tmp_path, O.synth_clips(1).astype(np.float32))
-    from audio_zen.utils import initialize_module
-    from audio_zen.inferencer.base_inferencer import BaseInferencer
+def _initialize_module(path, args):
+    """What a dotted [model] path means to the reference loader: import the module, instantiate the class with the args."""
+    module, cls = path.rsplit(".", 1)
+    return getattr(importlib.import_module(module), cls)(**args)
+
+
+def _load_model(model_config, checkpoint_path, device):
+    """The steps of the reference's _load_model: build from the TOML, load ``ckpt["model"]`` strictly, move, eval."""
+    model = _initialize_module(model_config["path"], model_config["args"])
+    ckpt = torch.load(checkpoint_path, map_location="cpu")
+    model.load_state_dict(ckpt["model"])
+    model.to(device)
+    model.eval()
+    return model, ckpt["epoch"]
+
+
+def test_reference_loader_builds_and_loads_the_dropin_class(tmp_path, built_lib, golden):
+    g = golden("reference_inferencer")
+    cfg, ckpt = _config(tmp_path)
     from fsnplus_b200.model import FullSubNet_Plus
-    m = initialize_module(cfg["model"]["path"], args=cfg["model"]["args"])
+    m = _initialize_module(cfg["model"]["path"], cfg["model"]["args"])
     assert isinstance(m, FullSubNet_Plus)
-    model, epoch = BaseInferencer._load_model(cfg["model"], ckpt, torch.device("cpu"))      # strict load_state_dict inside
+    model, epoch = _load_model(cfg["model"], ckpt, torch.device("cpu"))     # strict load_state_dict inside
     assert isinstance(model, FullSubNet_Plus) and epoch == 7 and not model.training
     assert sum(p.numel() for p in model.parameters()) == 8675102                           # SURVEY.md 8a
-    # same keys and shapes as the reference class built from the same TOML section
-    Plus, _ = ref_loader.model_classes()
-    ref_sd = Plus(**cfg["model"]["args"]).state_dict()
+    # same keys, in the same order, and shapes as the reference class built from the same TOML section
     sd = model.state_dict()
-    assert list(sd.keys()) == list(ref_sd.keys())
-    assert all(sd[k].shape == ref_sd[k].shape for k in sd)
+    assert list(sd.keys()) == list(g["state_dict_keys"])
+    assert all(list(sd[k].shape) == [d for d in s if d >= 0] for k, s in zip(sd, g["state_dict_shapes"]))
     x = torch.zeros(1, 1, 257, 10)
     with pytest.raises(RuntimeError, match="no CPU fallback"):
         model(x, x, x)
 
 
-@needs_ref
 @pytest.mark.gpu
 def test_reference_inferencer_runs_the_dropin_model_on_gpu(tmp_path, built_lib, golden):
-    """tools/inference.py:11-18 of the reference, verbatim: initialize_module(inferencer path) -> Inferencer(config, ckpt, out)()."""
-    g = golden("plus_default")
-    clips = O.synth_clips(2).astype(np.float32)                            # clip 0 is the golden clip
-    cfg, ckpt = _config(tmp_path, clips)
-    _, sf = ref_loader._stubs()
-    sf.written.clear()
-    from audio_zen.utils import initialize_module
-    inferencer_class = initialize_module(cfg["inferencer"]["path"], initialize=False)
-    inferencer = inferencer_class(cfg, ckpt, tmp_path / "out")
+    """The reference inferencer's loop, one clip per call: STFT -> model(mag, real, imag) -> decompress_cIRM x spectrum -> iSTFT
+    -> int16, with the drop-in model on the B200; every call has the shapes the reference inferencer used."""
+    from fsnplus_b200 import inference as H
     from fsnplus_b200.model import FullSubNet_Plus
-    assert isinstance(inferencer.model, FullSubNet_Plus) and inferencer.device.type == "cuda"
-    inferencer()
-    names = sorted(os.path.basename(k) for k in sf.written)
-    assert names == ["clip0.wav", "clip1.wav"]
-    key = [k for k in sf.written if k.endswith("clip0.wav")][0]
-    assert os.path.basename(os.path.dirname(key)) == "enhanced_0007"
-    pcm, rate = sf.written[key]
-    want = np.int16(0.8 * np.iinfo(np.int16).max * g["enhanced"][0] / np.max(np.abs(g["enhanced"][0])))     # base_inferencer.py:151-152
-    assert rate == 16000 and pcm.dtype == np.int16 and pcm.shape == want.shape
-    err = O.rel_l2(pcm.astype(np.float64), want.astype(np.float64))
-    print(f"\n[reference inferencer + drop-in model] int16 waveform vs all-reference pipeline: rel-L2 {err:.3e}, "
-          f"max |diff| {np.abs(pcm.astype(int) - want.astype(int)).max()} LSB")
-    assert err < 2e-3
+    from fsnplus_b200.tools import inference as T
+    g = golden("reference_inferencer")
+    clips = O.synth_clips(2).astype(np.float32)
+    cfg, ckpt = _config(tmp_path)
+    dev = torch.device("cuda:0")
+    model, epoch = _load_model(cfg["model"], ckpt, dev)
+    assert isinstance(model, FullSubNet_Plus) and epoch == 7
+    assert [os.path.basename(f) for f in g["files"]] == ["clip0.wav", "clip1.wav"]
+    assert all(os.path.dirname(f) == f"enhanced_{str(epoch).zfill(4)}" for f in g["files"])
+    ac = cfg["acoustics"]
+    stft_args = (ac["n_fft"], ac["hop_length"], ac["win_length"])
+    for i, clip in enumerate(clips):
+        noisy = torch.from_numpy(clip)[None].to(dev)
+        X = H.stft(noisy, *stft_args)
+        ins = (X.abs().unsqueeze(1), X.real.unsqueeze(1).contiguous(), X.imag.unsqueeze(1).contiguous())
+        with torch.no_grad():
+            crm = model(*ins)
+        assert [list(x.shape) for x in ins] + [list(crm.shape)] == g["model_calls"][i].tolist()
+        enhanced = H.istft(H.apply_cirm(crm, X), *stft_args, length=noisy.size(-1))[0].cpu().numpy()
+        pcm, want = T.to_int16(enhanced), g["pcm"][i]
+        assert pcm.dtype == np.int16 and pcm.shape == want.shape
+        err = O.rel_l2(pcm.astype(np.float64), want.astype(np.float64))
+        print(f"\n[reference inferencer loop + drop-in model] clip{i} int16 waveform vs all-reference inferencer: rel-L2 {err:.3e}, "
+              f"max |diff| {np.abs(pcm.astype(int) - want.astype(int)).max()} LSB")
+        assert err < 2e-3
